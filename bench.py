@@ -6,7 +6,7 @@ Metric: Mrays/s (whole job) for full-image renders of the synthetic "lego_render
 A "step" = one full image per GPU through the hot path (voxel query -> row packing -> fused pair MLPs -> colour MLP ->
 composite), ONE `render_full` call.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--sr 24] [--only main]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--sr 24] [--only main] [--dump-outputs DIR]
 
 N>1 is launched by torchrun (one rank per GPU, NCCL).  The JSON line of every N carries
   value / ms_per_step  WEAK scaling: N distinct camera poses (rolls about the view axis), rank g renders frame g, one all-gather of
@@ -18,6 +18,11 @@ N>1 is launched by torchrun (one rank per GPU, NCCL).  The JSON line of every N 
   scannet              BASELINE configs[4]: N=5M points (P=30), the same step with the sparse touched-rows gradient exchange, plus one
                        prune + probe + grow cycle (variable-length all-gather of the new points);
   cold, sr80           (N=1) first frame of a new point cloud (voxel grid + per-point table built inside the timed region); SR=80.
+
+`--dump-outputs DIR` writes what the last of the K timed steps of the main line returned (rank 0's frame) as DIR/<name>.npy, float32:
+the render_full outputs coarse_raycolor [1,R,3], coarse_is_background [1,R,1] and ray_mask [1,R] in full, and coarse_point_opacity
+[1,R,SR] for a fixed, seeded sample of DUMP_OPACITY_RAYS rays (their indices in coarse_point_opacity_rays.npy).  The scene, weights and
+rays are seeded: the same arguments give the same inputs on every run, so two builds can be compared output for output.
 
 `--impl reference` times the reference's own CPU path (the oracle port: oracle/query_oracle.c + oracle/shade_oracle.py, i.e. the
 reference's algorithm on the host cores) on a bounded, stratified sample of the same frame.  The oracle is used here ONLY as the
@@ -49,6 +54,7 @@ LAUNCHES_PER_STEP_TC = 11 + 5 + 1
 LAUNCHES_PER_STEP_FP32 = 11 + 1 + 1
 MMA_FLOPS = 2.0 * 128 * 256 * 16                      # one tcgen05.mma M128 N256 K16
 MMAS_PER_TILE = {True: 159, False: 201}               # frozen (k_shade_tc8) / general (k_shade_tc7) pair kernel, per 128-row tile
+DUMP_OPACITY_RAYS = 65536                             # the full [R,SR] opacity of an 800x800 frame alone is 61 MB
 
 
 def peaks():
@@ -304,17 +310,21 @@ def time_region(D, flush, fn, steps):
 
 def render_section(D, net, cam_list, rays_host, steps, warmup, flush, e2e=False):
     """Times `steps` frames.  rays_host: this rank's pinned [R,3] ray directions; cam_list: (campos, camrot, near, far, bg).
-    Resident mode: rays already on the device.  e2e mode: H2D of the rays and D2H of the colours inside every step."""
+    Resident mode: rays already on the device.  e2e mode: H2D of the rays and D2H of the colours inside every step.
+    Returns (ms, R, the render_full outputs of the last step)."""
     dev = D.dev
     R = rays_host.shape[0]
     rays_dev = rays_host.to(dev)
     gathered = [torch.empty((D.world, R, 3), dtype=torch.float32, device=dev) for _ in range(2)] if D.world > 1 else None
     out_host = torch.empty((R, 3), dtype=torch.float32).pin_memory()
+    last = {}
 
     def step(k):
         rd = rays_host.to(dev, non_blocking=True) if e2e else rays_dev
         with torch.no_grad():
             out = net.render_full(cam_list[0], rd, cam_list[1], cam_list[2], cam_list[3], cam_list[4])
+        if k == steps - 1:
+            last["out"] = out
         col = out["coarse_raycolor"][0]
         if D.world > 1:
             D.gather_async(col, gathered[k & 1])
@@ -333,9 +343,22 @@ def render_section(D, net, cam_list, rays_host, steps, warmup, flush, e2e=False)
         except PnbOverflow:                     # a scene denser than the workspace heuristic: the workspace has grown, warm up again
             if attempt == 1 or warmup == 0:
                 raise
+    last.clear()
     ms = time_region(D, flush, step, steps)
     net.check_errors()
-    return ms, R
+    return ms, R, last.get("out")
+
+
+def dump_outputs(out, directory):
+    """render_full outputs -> directory/<name>.npy (float32); coarse_point_opacity for a seeded sample of the rays."""
+    os.makedirs(directory, exist_ok=True)
+    arrays = {k: out[k].float().cpu().numpy() for k in ("coarse_raycolor", "coarse_is_background", "ray_mask")}
+    R = out["coarse_point_opacity"].shape[1]
+    rays = np.sort(np.random.RandomState(0).choice(R, min(R, DUMP_OPACITY_RAYS), replace=False))
+    arrays["coarse_point_opacity"] = out["coarse_point_opacity"][:, torch.from_numpy(rays).to(out["coarse_point_opacity"].device)].cpu().numpy()
+    arrays["coarse_point_opacity_rays"] = rays.astype(np.float32)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
 
 
 def main():
@@ -349,6 +372,8 @@ def main():
     ap.add_argument("--only", type=str, default="", help="comma list of sub-results to run besides the main line: strong,truck,train,scannet,cold,sr80 (default: all)")
     ap.add_argument("--precision", type=str, default="bf16x3", help="bf16x3 (tcgen05, default) | fp32 (CUDA cores)")
     ap.add_argument("--frozen", type=int, default=1, help="1 (default): frozen-cloud pair kernel k_shade_tc8 (point-only layer-1 inputs hoisted per point) | 0: general kernel k_shade_tc7")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write the outputs of the last timed step of the main line to DIR/<name>.npy (float32, rank 0)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -384,10 +409,13 @@ def main():
     # share their host, and a stalled launching thread occasionally adds milliseconds to a region that has nothing to do with the GPU
     # work - the repeat makes such a run recognisable
     regions = []
-    for _ in range(2):
+    for i in range(2):
         t_w0 = time.time()
-        ms_i, R = render_section(D, net, cam, mine, args.steps, 0, flush)
+        ms_i, R, out_i = render_section(D, net, cam, mine, args.steps, 0, flush)
         regions.append((ms_i, t_w0, time.time()))
+        if i == 0 and args.dump_outputs and rank == 0:
+            dump_outputs(out_i, args.dump_outputs)
+        del out_i
     ms_res, t_w0, t_w1 = regions[0]
     clocks = sampler.stop(t_w0, t_w1) if sampler else None
     # workload counters (oracle-independent: the library's own device counters)
@@ -449,7 +477,7 @@ def main():
         net.check_errors()
 
     # ---------------- e2e: host buffers, H2D of the rays + D2H of the colours inside the timed region
-    ms_e2e, _ = render_section(D, net, cam, mine, args.steps, 2, flush, e2e=True)
+    ms_e2e, _, _ = render_section(D, net, cam, mine, args.steps, 2, flush, e2e=True)
 
     total_rays = R * world * args.steps
     value = total_rays / (ms_res * 1e-3) / 1e6
@@ -467,7 +495,7 @@ def main():
     if "strong" in want:
         mine_s = dirs_cam[rank::world].contiguous().pin_memory()
         cam0 = (list(cfg.campos), torch.eye(3), cfg.near, cfg.far, bg)
-        ms_s, Rs = render_section(D, net, cam0, mine_s, args.steps, W, flush)
+        ms_s, Rs, _ = render_section(D, net, cam0, mine_s, args.steps, W, flush)
         sub["strong"] = dict(value=R_img * args.steps / (ms_s * 1e-3) / 1e6, unit="Mrays/s", ms_per_frame=ms_s / args.steps,
                              rays_per_rank=Rs, what="one 800x800 frame, ray i -> rank i %% %d, all-gather of the [R/N,3] tiles inside the timed "
                              "region (side stream, double-buffered)" % world)
@@ -490,7 +518,7 @@ def main():
         cfg80 = scene.CONFIGS["lego_render"]
         cfg80.SR = 80
         net80, _, _ = harness.build_model(cfg80, dev, seed=0, alpha_bias=3.0, pnb_precision=args.precision, pnb_frozen=args.frozen)
-        ms80, _ = render_section(D, net80, cam, mine, 5, W, flush)
+        ms80, _, _ = render_section(D, net80, cam, mine, 5, W, flush)
         sub["sr80"] = dict(value=R_img * 5 / (ms80 * 1e-3) / 1e6, unit="Mrays/s", ms_per_frame=ms80 / 5)
         cfg80.SR = args.sr
         del net80
@@ -502,7 +530,7 @@ def main():
         tdirs = scene.make_rays(tcfg)["raydir"][0]
         tmine = tdirs[rank::world].contiguous().pin_memory()
         tcam = (list(tcfg.campos), torch.eye(3), tcfg.near, tcfg.far, bg)
-        ms_t, Rt = render_section(D, tnet, tcam, tmine, 5, W, flush)
+        ms_t, Rt, _ = render_section(D, tnet, tcam, tmine, 5, W, flush)
         tq = tnet.neural_points.querier.run_query(tnet.neural_points.xyz.detach(), tmine.to(dev), tcam[0], tcam[2], tcam[3], want_counters=True).counters
         sub["truck"] = dict(value=tdirs.shape[0] * 5 / (ms_t * 1e-3) / 1e6, unit="Mrays/s", ms_per_frame=ms_t / 5, rays_per_rank=Rt,
                             workload="truck_8gpu: 960x540, N=2000000 points, kernel_size 5, vsize 0.002, SR=24, one frame interleave-sharded x%d" % world,

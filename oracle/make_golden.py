@@ -159,10 +159,55 @@ def golden_output_keys():
     print("output_keys:", {m: sorted(v) for m, v in res.items()})
 
 
+def _param_names(fn):
+    import inspect
+    return [p.name for p in inspect.signature(fn).parameters.values() if p.kind in (p.POSITIONAL_OR_KEYWORD, p.KEYWORD_ONLY)]
+
+
+def golden_reference_api():
+    """The parts of the reference's interface that the drop-in seams of INTEGRATION.md must match, as the reference's own classes report
+    them: method parameter names, the argparse namespace of the shipped flags, the aggregator's state-dict layout (in order) and the key
+    set of its evaluation-mode forward.  tests/test_reference_contract.py checks pointnerf_b200 against this file."""
+    import json
+    ref_shim.install()
+    from models.neural_points.point_query import lighting_fast_querier as RefQuerier
+    from models.neural_points.neural_points import NeuralPoints as RefPoints
+    from models.neural_points_volumetric_model import NeuralPointsRayMarching as RefMarch
+    sig = {}
+    for cls, names in ((RefQuerier, ("__init__", "query_points", "get_hyperparameters", "clean_up")),
+                       (RefPoints, ("prune", "grow_points", "set_points")), (RefMarch, ("forward",))):
+        for n in names:
+            sig["%s.%s" % (cls.__name__, n)] = _param_names(getattr(cls, n))
+    cfg = scene.CONFIGS["tiny"]
+    net, agg, npts, pts, opt = build_reference_net(cfg, 4.0)
+    rays = scene.make_rays(cfg, scene.centre_patch(cfg, 12))
+    with torch.no_grad():
+        out = net(rays["campos"], rays["raydir"], bg_color=rays["bg_color"], camrotc2w=rays["camrotc2w"], pixel_idx=rays["pixel_idx"],
+                  near=rays["near"], far=rays["far"], h=rays["h"], w=rays["w"], intrinsic=rays["intrinsic"])
+    res = dict(signatures=sig, opt=vars(opt),
+               aggregator_state_dict=[[k, list(v.shape), str(v.dtype).replace("torch.", "")] for k, v in agg.state_dict().items()],
+               net_state_dict_keys=sorted(net.state_dict().keys()),
+               forward_eval_keys=sorted(k for k, v in out.items() if v is not None))
+    with open(os.path.join(OUT, "reference_api.json"), "w") as f:
+        json.dump(res, f, indent=1, sort_keys=True)
+    # positional_encoding of models/helpers/networks.py on a seeded input, for the (freqs, ori) pairs the hot path uses
+    from models.helpers.networks import positional_encoding
+    g = torch.Generator().manual_seed(0)
+    x = torch.randn(7, 5, generator=g)
+    fx = dict(x=x.numpy())
+    for freqs, ori in ((3, False), (5, False), (4, True)):
+        fx["pe_%d_%d" % (freqs, int(ori))] = positional_encoding(x, freqs, ori=ori).numpy()
+    np.savez_compressed(os.path.join(OUT, "positional_encoding.npz"), **fx)
+    print("reference_api:", len(sig), "signatures,", len(res["opt"]), "options")
+
+
 if __name__ == "__main__":
     assert ref_shim.available(), "needs /root/reference"
     if len(sys.argv) > 1 and sys.argv[1] == "keys":
         golden_output_keys()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "api":
+        golden_reference_api()
         sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "order1":
         tiny = scene.CONFIGS["tiny"]
@@ -177,3 +222,4 @@ if __name__ == "__main__":
     golden_hyper()
     golden_checkpoint_layout()
     golden_output_keys()
+    golden_reference_api()

@@ -1,13 +1,13 @@
 """CPU: pins oracle/shade_oracle.py against numbers produced by the reference's own Python
 (PointAggregator / NeuralPointsRayMarching / ray_march run unmodified on CPU, oracle/make_golden.py),
-forward values and autograd gradients, and -- when the reference tree is present -- directly."""
+forward values and autograd gradients."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim, shade_oracle
+from oracle import shade_oracle
 from pointnerf_b200 import scene
 
 
@@ -55,10 +55,9 @@ def test_fill_invalid(golden_dir):
     assert torch.all(out["coarse_point_opacity"][~mask] == 0)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
-def test_positional_encoding_matches_reference():
-    ref_shim.install()
-    from models.helpers.networks import positional_encoding as ref_pe
-    x = torch.randn(7, 5)
+def test_positional_encoding_matches_reference(golden_dir):
+    """vs the reference's models/helpers/networks.py positional_encoding on a seeded input (oracle/make_golden.py)."""
+    fx = np.load(os.path.join(golden_dir, "positional_encoding.npz"))
+    x = torch.from_numpy(fx["x"])
     for freqs, ori in ((3, False), (5, False), (4, True)):
-        assert torch.equal(ref_pe(x, freqs, ori=ori), shade_oracle.positional_encoding(x, freqs, ori=ori))
+        assert torch.equal(torch.from_numpy(fx["pe_%d_%d" % (freqs, int(ori))]), shade_oracle.positional_encoding(x, freqs, ori=ori))
