@@ -53,13 +53,15 @@ struct ShadeTcParams {
     int hbar_cap;
     int* err;
     int dbg_no_weights;          // timing experiment only: the loader signals the ring without copying (results are garbage)
-    int dbg_flags;               // bit 1: v6 issuer classifies its waits with non-blocking probes (profiling)
+    int dbg_flags;               // bit 0: cycle accounting of block 0; bit 2: per-CTA cycles; bit 3: v8 non-deferred last epilogue;
+                                 // bit 4: v8 static tile schedule instead of the tile queue
     const unsigned char* vcnt;   // v7 row packing: neighbours per PACKED position [n_valid] (vcntp of k_pack_quads)
     const uint32_t* vorder;      // v7: valid-sample index of every packed position [n_valid]
     const uint32_t* quad_first;  // v7: first valid sample of every 32-row quadrant [n_quads + 1]
     const int* pack_cnt;         // v7: [0] = n_quads
     const float* pre;            // v8: per-point hoisted layer-1 pre-activation [N][256] (k_point_pre)
     int hbar_fmt;                // 0: hbar[n_valid][256] fp32;  1: bf16 hi/lo A-operand blocks of k_color_tc2 (per 128 samples: 8 K blocks x {hi,lo} x [128x32])
+    int* tile_ctr;               // v8: tile queue, next 128-row tile to hand out (= pack_cnt + 1, zeroed by k_pack_scan)
 };
 __device__ __forceinline__ void prof_add(const ShadeTcParams& p, int slot, long long cyc) {
     if ((p.dbg_flags & 1) && blockIdx.x == 0) atomicAdd(reinterpret_cast<unsigned long long*>(p.err) + 1 + slot, (unsigned long long)cyc);
@@ -363,7 +365,7 @@ __global__ void __launch_bounds__(256) k_pack_quads(pnb_query_t q, int cap, uint
     if (lane == 0) sc_quads[sc] = (uint32_t)nq;
 }
 // exclusive scan of the per-super-chunk quadrant counts (one block): sc_quads[0 .. n_sc] (last = total), total -> pack_cnt[0],
-// sentinel quad_first[n_quads] = n_valid
+// sentinel quad_first[n_quads] = n_valid; also zeroes the tile queue counter pack_cnt[1] of k_shade_tc8 (no extra launch per call)
 __global__ void __launch_bounds__(1024) k_pack_scan(pnb_query_t q, int cap, uint32_t* __restrict__ sc_quads, uint32_t* __restrict__ quad_first,
                                                     int* __restrict__ pack_cnt) {
     __shared__ uint32_t wsum[32];
@@ -384,7 +386,7 @@ __global__ void __launch_bounds__(1024) k_pack_scan(pnb_query_t q, int cap, uint
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, iv, d); if (lane >= d) iv += t; }
         wsum[lane] = iv - v;
-        if (lane == 31) { pack_cnt[0] = (int)iv; quad_first[iv] = (uint32_t)n_valid; sc_quads[n_sc] = iv; }
+        if (lane == 31) { pack_cnt[0] = (int)iv; pack_cnt[1] = 0; quad_first[iv] = (uint32_t)n_valid; sc_quads[n_sc] = iv; }
     }
     __syncthreads();
     uint32_t run = wsum[w] + incl - sum;
@@ -405,13 +407,13 @@ __global__ void __launch_bounds__(256) k_pack_place(pnb_query_t q, int cap, cons
 // <= 8 lanes, first lane st); the last row of a sample (swrite) holds the sums and writes h-bar.
 // EARLY (v8): ALL chunks of this warp are read into registers first and `drain_bar` is signalled right away - the accumulator region
 // is then free for layer 2 of the next tile ~2 k cycles after the last MMA instead of after the whole reduction (~10 k).
+// bias / wa: bias of block3.2 and the alpha weight (k_shade_tc8 passes its shared-memory copies: plain loads, no __ldg).
 // O1: agg_intrp_order == 1 as a COMPILE-TIME flag (as a run-time flag ptxas if-converted the order-1 dot product: 16 extra loads + FMAs per
 // chunk executed speculatively on the shipped order-2 path, seen in the ncu source page).
 template <int NG, int NCHUNK, bool EARLY = false, bool O1 = false>
-__device__ __forceinline__ float last_chunks_packed(const ShadeTcParams& p, uint32_t accb, int G, float wrow, int st, bool swrite, int sidx, int lane,
-                                                    uint64_t* drain_bar = nullptr) {
+__device__ __forceinline__ float last_chunks_packed(const ShadeTcParams& p, const float* bias, const float* wa, uint32_t accb, int G, float wrow, int st,
+                                                    bool swrite, int sidx, int lane, uint64_t* drain_bar = nullptr) {
     using namespace tc;
-    const float* bias = p.bias[3];
     constexpr bool order1 = O1;
     float apart = 0.f;
     uint32_t vv[EARLY ? NCHUNK : 2][16];
@@ -436,7 +438,7 @@ __device__ __forceinline__ float last_chunks_packed(const ShadeTcParams& p, uint
         float z[16];
 #pragma unroll
         for (int e4 = 0; e4 < 4; ++e4) {
-            const float4 bb = __ldg(reinterpret_cast<const float4*>(bias + c0) + e4), ww = __ldg(reinterpret_cast<const float4*>(p.wa + c0) + e4);
+            const float4 bb = reinterpret_cast<const float4*>(bias + c0)[e4], ww = reinterpret_cast<const float4*>(wa + c0)[e4];
             const float bq[4] = {bb.x, bb.y, bb.z, bb.w}, wq[4] = {ww.x, ww.y, ww.z, ww.w};
 #pragma unroll
             for (int e1 = 0; e1 < 4; ++e1) {
@@ -451,7 +453,7 @@ __device__ __forceinline__ float last_chunks_packed(const ShadeTcParams& p, uint
         for (int e = 0; e < 16; ++e) z[e] = seg_scan8(z[e], lane, st);
         if (order1) {       // agg_intrp_order 1: the alpha dot product runs over the K-aggregated feature (complete on the sample's last row)
 #pragma unroll
-            for (int e = 0; e < 16; ++e) apart = fmaf(z[e], __ldg(p.wa + c0 + e), apart);
+            for (int e = 0; e < 16; ++e) apart = fmaf(z[e], wa[c0 + e], apart);
         }
         if (swrite) {
             if (p.hbar_fmt) {       // the colour kernel's operand image (bf16 hi / lo, core-matrix layout): two 16-byte rows each
@@ -478,15 +480,14 @@ __device__ __forceinline__ float last_chunks_packed(const ShadeTcParams& p, uint
 // One 16-column chunk of the last epilogue from REGISTERS (the deferred form of last_chunks_packed<.., EARLY = true>: identical
 // arithmetic in identical order, so the two forms give bit-identical h-bar / alpha sums): columns c0 .. c0+15 of this lane's row in v.
 template <bool O1>
-__device__ __forceinline__ void last_chunk_from_regs(const ShadeTcParams& p, int c0, const uint32_t* v, float wrow, int st, bool swrite, int sidx, int lane,
-                                                     float& apart) {
+__device__ __forceinline__ void last_chunk_from_regs(const ShadeTcParams& p, const float* bias, const float* wa, int c0, const uint32_t* v, float wrow, int st,
+                                                     bool swrite, int sidx, int lane, float& apart) {
     using namespace tc;
-    const float* bias = p.bias[3];
     constexpr bool order1 = O1;
     float z[16];
 #pragma unroll
     for (int e4 = 0; e4 < 4; ++e4) {
-        const float4 bb = __ldg(reinterpret_cast<const float4*>(bias + c0) + e4), ww = __ldg(reinterpret_cast<const float4*>(p.wa + c0) + e4);
+        const float4 bb = reinterpret_cast<const float4*>(bias + c0)[e4], ww = reinterpret_cast<const float4*>(wa + c0)[e4];
         const float bq[4] = {bb.x, bb.y, bb.z, bb.w}, wq[4] = {ww.x, ww.y, ww.z, ww.w};
 #pragma unroll
         for (int e1 = 0; e1 < 4; ++e1) {
@@ -501,7 +502,7 @@ __device__ __forceinline__ void last_chunk_from_regs(const ShadeTcParams& p, int
     for (int e = 0; e < 16; ++e) z[e] = seg_scan8(z[e], lane, st);
     if (order1) {
 #pragma unroll
-        for (int e = 0; e < 16; ++e) apart = fmaf(z[e], __ldg(p.wa + c0 + e), apart);
+        for (int e = 0; e < 16; ++e) apart = fmaf(z[e], wa[c0 + e], apart);
     }
     if (swrite) {
         if (p.hbar_fmt) {
@@ -695,7 +696,7 @@ __global__ void __launch_bounds__(tc7::NTHR, 1) k_shade_tc7(ShadeTcParams p) {
                 const int sidx = qr.live ? (int)p.vorder[sm.qfirst[tf & 1][qw] + qr.j] : 0;
                 const bool swrite = qr.is_end && sidx < n_valid;
                 const float wrow = sm.wc[tf & 1][row];
-                const float apart = last_chunks_packed<4, 4, false, O1>(p, tP + tlane, 2 + part, wrow, qr.st, swrite, sidx, lane);
+                const float apart = last_chunks_packed<4, 4, false, O1>(p, p.bias[3], p.wa, tP + tlane, 2 + part, wrow, qr.st, swrite, sidx, lane);
                 tc_fence_before();
                 sm.alpha_part[part][row] = apart;
                 named_bar_sync(2, tc7::NBUILD);
@@ -756,7 +757,7 @@ __global__ void __launch_bounds__(tc7::NTHR, 1) k_shade_tc7(ShadeTcParams p) {
                 tc_fence_after();
                 const QuadRow qr = quad_row(sm.qhead[t & 1][quad], (int)sm.qtotal[t & 1][quad], lane);
                 const int sidx = qr.live ? (int)p.vorder[sm.qfirst[t & 1][quad] + qr.j] : 0;
-                const float apart = last_chunks_packed<4, 4, false, O1>(p, tP + tlane, grp, sm.wc[t & 1][erow], qr.st, qr.is_end && sidx < n_valid, sidx, lane);
+                const float apart = last_chunks_packed<4, 4, false, O1>(p, p.bias[3], p.wa, tP + tlane, grp, sm.wc[t & 1][erow], qr.st, qr.is_end && sidx < n_valid, sidx, lane);
                 tc_fence_before();
                 atomicAdd(&sm.alpha_e[erow], apart);
                 __syncwarp();
@@ -814,8 +815,12 @@ struct Smem {
     float wc[NWC][tc::TM];
     float alpha_part[2][NGRP][tc::TM];    // [tile parity][epilogue group] partial alpha dot products (own slot each: summed in a fixed order)
     int prow[2][tc::TM];                  // point index of every row (-1: unused row)
+    alignas(16) float bias[3][256];       // copies of the layer 2..4 biases and the alpha weight: the epilogues read them per chunk as
+    alignas(16) float wa[256];            // warp-broadcast LDS.128 instead of __ldg (LSU data pipe shared with tcgen05.ld/st and the gather)
+    int tile_slot[2];                     // tile index of this CTA's tile t in [t & 1] (-1: no tile left), written by builder warp 0
     uint32_t qhead[NWC][4], qfirst[NWC][4], qtotal[NWC][4];
-    uint64_t bar_full[NSTAGE], bar_empty[NSTAGE], bar_a1_ready, bar_a1_free, bar_acc_full, bar_final, bar_alpha, bar_drain, bar_kblk[8], bar_prow[2];
+    uint64_t bar_full[NSTAGE], bar_empty[NSTAGE], bar_a1_ready, bar_a1_free, bar_acc_full, bar_final, bar_alpha, bar_drain, bar_kblk[8], bar_prow[2],
+             bar_tile[2];
     uint32_t tmem_base;
 };
 }  // namespace tc8
@@ -966,7 +971,7 @@ struct Tc8Pf {                                    // chunks of `pre` in flight p
     }
 };
 
-// One epilogue layer of a warp: chunks grp, grp+NGRP, ... (16 accumulator columns each): accumulator -> (+ bias or + pre[point]) ->
+// One epilogue layer of a warp: chunks grp, grp+NGRP, ... (16 accumulator columns each): accumulator -> (+ bias (shared memory) or + pre[point]) ->
 // LeakyReLU -> bf16 hi/lo -> the same columns, one mbarrier arrive per warp and chunk.
 template <bool FIRST, bool COOP, class SmemT, class PfT>
 __device__ __forceinline__ void tc8_epi_layer(SmemT& sm, uint32_t accb, int grp, const float* __restrict__ bias, PfT& pfs, unsigned char* xp) {
@@ -983,7 +988,7 @@ __device__ __forceinline__ void tc8_epi_layer(SmemT& sm, uint32_t accb, int grp,
         if (FIRST) pfs.fetch(i % PF, xp, lane, b4);
         else {
 #pragma unroll
-            for (int e = 0; e < 4; ++e) b4[e] = __ldg(reinterpret_cast<const float4*>(bias + c0) + e);
+            for (int e = 0; e < 4; ++e) b4[e] = reinterpret_cast<const float4*>(bias + c0)[e];     // shared-memory copy
         }
         if (FIRST && i + PF < NCH) pfs.load(i % PF, g + NGRP * PF);
         tmem_ld_wait();
@@ -1020,6 +1025,17 @@ __device__ __forceinline__ void tc8_epi_layer(SmemT& sm, uint32_t accb, int grp,
 // XF: layers are queued back to back (tcgen05.mma execute in issue order: a layer's accumulator region is the previous layer's dead operand
 // region, so the issuer need not wait for the previous layer's completion barrier - only for the per-K-block operand barriers), and layer 3
 // issues its extras K block (operand from shared memory, independent of the layer-2 epilogue) FIRST, into the layer turn-around bubble.
+// TILE QUEUE: the tiles are handed out in increasing order by one device counter (p.tile_ctr, zeroed by k_pack_scan of the same call), so
+// a CTA that runs slower simply takes fewer tiles (static striding made the kernel as long as its slowest CTA; dbg bit 4 keeps it for A/B).
+// Builder warp 0 takes tile t of this CTA right after bar_a1_free(t-1) (and, DEFER, bar_drain(t-2)), i.e. about one tile ahead, writes it -
+// or -1 when none is left - into tile_slot[t & 1] and arrives on bar_tile[t & 1].  The other builder warps and the loader wait on bar_tile;
+// the issuer and the epilogue warps read the slot after bar_a1_ready(t) / bar_prow(t), which the builders arrive on also for the -1 (then
+// without an operand) so that every role leaves its loop at the same t.  No waiter is overtaken by two phase completions, and the slot is
+// not rewritten before every reader of tile t has read it: bar_tile[t & 1] / tile_slot[t & 1] next change for tile t+2, after builder warp 0
+// has seen bar_a1_free(t+1) - the issuer has then taken tile t+1 (so it read slot t), the loader has streamed the layer-1 weights of tile
+// t+1 (so it passed its bar_tile(t) wait), and the other builder warps have arrived on bar_a1_ready(t+1) (so they passed theirs).  The
+// epilogue warps read slot t before their drain of tile t: DEFER, warp 0 also waits for bar_drain(t) first; non-deferred, it has waited for
+// bar_alpha(t) one iteration earlier (finish_sigma).  bar_a1_ready / bar_prow keep their previous arguments; the -1 is their last phase.
 template <int NSTAGE, bool COOP, bool DEFER, bool O1 = false, int SCHED = 0, int PFN = 3, bool UNI = true, bool XF = true>
 __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shade_tc8(ShadeTcParams p) {
     using SmemT = tc8::Smem<NSTAGE, COOP>;
@@ -1036,7 +1052,8 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
     const int n_valid = min(q.counters[PNB_QC_N_VALID], p.hbar_cap);
     const int n_quads = p.pack_cnt[0];
     const int n_tiles = (n_quads + 3) >> 2;
-    const int my_tiles = n_tiles > (int)blockIdx.x ? (n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+    const bool static_sched = (p.dbg_flags & 16) != 0;      // tile t of a CTA = blockIdx.x + t * gridDim.x (A/B against the queue)
+    int n_done = 0;                                          // tiles this CTA processed (per-CTA statistics, dbg bit 2)
     constexpr int NEPI_WARPS = tc8::NEPI_WARPS;
     constexpr int W_BUILD = NEPI_WARPS, W_LOAD = W_BUILD + tc8::NBUILD / 32, W_ISSUE = W_LOAD + 1;
     // last epilogue: 16 chunks over the NGRP epilogue warps + 1 builder warp of a quadrant; the builder warp takes group 0
@@ -1054,8 +1071,14 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
         for (int c = 0; c < 8; ++c) mbar_init(&sm.bar_kblk[c], 4 * 2);   // 4 quadrant warps x 2 chunks of 16 columns, one arrive per warp
         mbar_init(&sm.bar_prow[0], tc8::NBUILD / 32);
         mbar_init(&sm.bar_prow[1], tc8::NBUILD / 32);
+        mbar_init(&sm.bar_tile[0], 1);
+        mbar_init(&sm.bar_tile[1], 1);
         mbar_fence_init();
         if (blockIdx.x == 0 && q.counters[PNB_QC_N_VALID] > p.hbar_cap) atomicExch(p.err, 9);
+    }
+    for (int i = tid; i < 4 * 256; i += (int)blockDim.x) {
+        if (i < 3 * 256) sm.bias[i >> 8][i & 255] = __ldg(p.bias[1 + (i >> 8)] + (i & 255));
+        else sm.wa[i - 3 * 256] = __ldg(p.wa + (i - 3 * 256));
     }
     if (warp == W_ISSUE) tmem_alloc<512>(&sm.tmem_base);
     tc_fence_before();
@@ -1085,11 +1108,12 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
         const uint32_t ahi_lo = uni32(desc_lo<LAYOUT>(smem_u32(sm.a_hi))), alo_lo = uni32(desc_lo<LAYOUT>(smem_u32(sm.a_lo)));
         const uint32_t xeh_lo0 = uni32(desc_lo<LAYOUT_NONE>(smem_u32(sm.xe_hi[0]))), xel_lo0 = uni32(desc_lo<LAYOUT_NONE>(smem_u32(sm.xe_lo[0])));
         const uint32_t uP = uni32(sm.tmem_base), uQ = uP + 256u;
-        const int n_my = (int)uni32((uint32_t)my_tiles);
         constexpr uint32_t KADV = kstep_adv16<LAYOUT>();
         uint32_t s = 0, ph = 0, c_acc = 0, c_pack = 0;
         bool ok = true;
-        for (int t = 0; t < n_my && ok; ++t) {
+        for (int t = 0; ok; ++t) {
+            if (!uni(TW(3, mbar_wait(&sm.bar_a1_ready, (uint32_t)t & 1u, p.err, 93)))) { ok = false; break; }
+            if ((int)uni32((uint32_t)sm.tile_slot[t & 1]) < 0) break;           // no tile left (the builders' end signal)
             const uint32_t xeh_lo = xeh_lo0 + (uint32_t)(t & 1) * (XE >> 4), xel_lo = xel_lo0 + (uint32_t)(t & 1) * (XE >> 4);
             for (int l = 0; l < 4 && ok; ++l) {
                 const uint32_t acc = (l & 1) ? uP : uQ;
@@ -1098,7 +1122,6 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
                     if (l > 0) { if (!uni(TW(1, mbar_wait(&sm.bar_acc_full, c_acc & 1u, p.err, 92)))) { ok = false; break; } ++c_acc; }
                     else if (t > 0) { if (!uni(TW(2, mbar_wait(&sm.bar_final, (uint32_t)(t - 1) & 1u, p.err, 92)))) { ok = false; break; } }
                 }
-                if (l == 0) { if (!uni(TW(3, mbar_wait(&sm.bar_a1_ready, (uint32_t)t & 1u, p.err, 93)))) { ok = false; break; } }
                 if (l == 1 && t > 0) { if (!uni(TW(4, mbar_wait(&sm.bar_drain, (uint32_t)(t - 1) & 1u, p.err, 94)))) { ok = false; break; } }
                 tc_fence_after();
                 const int nkb = l == 0 ? tc8::NKB1 : nkb_of(l);
@@ -1147,22 +1170,25 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
     } else if (warp == W_LOAD) {
         // ============================================================ weight ring: one K block (hi + lo image, 32 KB) per stage
         if (lane == 0) {
-            const uint32_t total = (uint32_t)my_tiles * tc8::STAGES_PER_TILE;
-            uint32_t s = 0, ph = 0, j = 0;
-            for (uint32_t n = 0; n < total; ++n) {
-                if (!TW(0, mbar_wait(&sm.bar_empty[s], ph ^ 1u, p.err, 91))) break;
-                uint32_t blk = j < (uint32_t)tc8::NKB1 ? (uint32_t)tc8::KB1_FIRST + j : 9u + (j - (uint32_t)tc8::NKB1);
-                // XF: layer 3 (stages NKB1 + 8 .. NKB1 + 16 of a tile, weight blocks 17 .. 25) takes its extras block (25) FIRST
-                if (XF && j >= (uint32_t)tc8::NKB1 + 8u && j < (uint32_t)tc8::NKB1 + 17u) blk = j == (uint32_t)tc8::NKB1 + 8u ? 25u : blk - 1u;
-                if (p.dbg_no_weights) mbar_arrive(&sm.bar_full[s]);
-                else {
-                    mbar_arrive_expect_tx(&sm.bar_full[s], tc8::STAGE);
-                    const unsigned char* src = p.wimg + (size_t)blk * tc8::STAGE;
-                    bulk_g2s(sm.b[s], src, IMG, &sm.bar_full[s]);
-                    bulk_g2s(sm.b[s] + IMG, src + IMG, IMG, &sm.bar_full[s]);
+            uint32_t s = 0, ph = 0;
+            bool ok = true;
+            for (int t = 0; ok; ++t) {
+                // tile t exists?  (published by builder warp 0 right after it took the tile, a layer or more ahead of the ring)
+                if (!mbar_wait(&sm.bar_tile[t & 1], (uint32_t)(t >> 1) & 1u, p.err, 106) || sm.tile_slot[t & 1] < 0) break;
+                for (uint32_t j = 0; j < (uint32_t)tc8::STAGES_PER_TILE; ++j) {
+                    if (!TW(0, mbar_wait(&sm.bar_empty[s], ph ^ 1u, p.err, 91))) { ok = false; break; }
+                    uint32_t blk = j < (uint32_t)tc8::NKB1 ? (uint32_t)tc8::KB1_FIRST + j : 9u + (j - (uint32_t)tc8::NKB1);
+                    // XF: layer 3 (stages NKB1 + 8 .. NKB1 + 16 of a tile, weight blocks 17 .. 25) takes its extras block (25) FIRST
+                    if (XF && j >= (uint32_t)tc8::NKB1 + 8u && j < (uint32_t)tc8::NKB1 + 17u) blk = j == (uint32_t)tc8::NKB1 + 8u ? 25u : blk - 1u;
+                    if (p.dbg_no_weights) mbar_arrive(&sm.bar_full[s]);
+                    else {
+                        mbar_arrive_expect_tx(&sm.bar_full[s], tc8::STAGE);
+                        const unsigned char* src = p.wimg + (size_t)blk * tc8::STAGE;
+                        bulk_g2s(sm.b[s], src, IMG, &sm.bar_full[s]);
+                        bulk_g2s(sm.b[s] + IMG, src + IMG, IMG, &sm.bar_full[s]);
+                    }
+                    if (++s == (uint32_t)NSTAGE) { s = 0; ph ^= 1u; }
                 }
-                if (++s == (uint32_t)NSTAGE) { s = 0; ph ^= 1u; }
-                if (++j == (uint32_t)tc8::STAGES_PER_TILE) j = 0;
             }
         }
     } else if (warp > W_ISSUE) {
@@ -1176,12 +1202,13 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
         bool ok = true;
         // sigma of a tile = softplus(alpha dot product - 1) summed over the rows of a sample; the dot product is this warp's partial sum + the
         // epilogue warps' (bar_alpha), added in a fixed order
+        const float ba = __ldg(p.ba);
         auto finish_sigma = [&](int tf, float apart, float wrow, int st, bool swrite, int sidx) -> bool {
             if (!TW(12, mbar_wait(&sm.bar_alpha, (uint32_t)tf & 1u, p.err, 100))) return false;
             float a = apart;
 #pragma unroll
             for (int gq = 0; gq < NGRP; ++gq) a += sm.alpha_part[tf & 1][gq][row];          // fixed order: deterministic
-            a += __ldg(p.ba) - 1.0f;
+            a += ba - 1.0f;
             const float sp = a > 20.f ? a : log1pf(expf(a));
             const float zz = O1 ? sp : seg_scan8(sp * wrow, lane, st);      // (order 1: see k_shade_tc7)
             if (swrite) p.sigma[sidx] = zz;
@@ -1190,12 +1217,28 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
         float pd_apart = 0.f, pd_wrow = 0.f;          // DEFER: this warp's share of the tile drained one iteration ago (sigma still to be finished)
         int pd_st = 0, pd_sidx = 0;
         bool pd_sw = false;
-        for (int t = 0; t <= my_tiles && ok; ++t) {
-            if (t < my_tiles) {
-                const int tile = (int)blockIdx.x + t * (int)gridDim.x;
-                if (t > 0 && !TW(8, mbar_wait(&sm.bar_a1_free, (uint32_t)(t - 1) & 1u, p.err, 97))) { ok = false; break; }
-                // DEFER: the per-tile slots (qhead / qfirst / qtotal / wc, parity t & 1) were last read when tile t-2 was drained
-                if (DEFER && t > 1 && !mbar_wait(&sm.bar_drain, (uint32_t)(t - 2) & 1u, p.err, 103)) { ok = false; break; }
+        int t = 0;
+        for (;; ++t) {
+            if (t > 0 && !TW(8, mbar_wait(&sm.bar_a1_free, (uint32_t)(t - 1) & 1u, p.err, 97))) { ok = false; break; }
+            // DEFER: the per-tile slots (tile_slot / qhead / qfirst / qtotal / wc, parity t & 1) were last read when tile t-2 was drained
+            if (DEFER && t > 1 && !mbar_wait(&sm.bar_drain, (uint32_t)(t - 2) & 1u, p.err, 103)) { ok = false; break; }
+            int tile;                                     // this CTA's tile t, -1: none left
+            if (qw == 0) {
+                int v = 0;
+                if (lane == 0) {
+                    v = static_sched ? (int)blockIdx.x + t * (int)gridDim.x : atomicAdd(p.tile_ctr, 1);
+                    if (v >= n_tiles) v = -1;
+                    sm.tile_slot[t & 1] = v;
+                    mbar_arrive(&sm.bar_tile[t & 1]);
+                }
+                tile = __shfl_sync(0xffffffffu, v, 0);
+            } else {
+                if (!mbar_wait(&sm.bar_tile[t & 1], (uint32_t)(t >> 1) & 1u, p.err, 105)) { ok = false; break; }
+                tile = sm.tile_slot[t & 1];
+            }
+            if (tile < 0) {                               // end: wake the issuer and the epilogue warps, which read the slot
+                if (lane == 0) { mbar_arrive(&sm.bar_a1_ready); mbar_arrive(&sm.bar_prow[t & 1]); }
+            } else {
                 const int qd = tile * 4 + qw;
                 uint32_t first = 0, nsamp = 0;
                 if (qd < n_quads) { first = p.quad_first[qd]; nsamp = p.quad_first[qd + 1] - first; }
@@ -1227,7 +1270,7 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
                 const int sidx = qr.live ? (int)p.vorder[sm.qfirst[tf & 1][qw] + qr.j] : 0;
                 const bool swrite = qr.is_end && sidx < n_valid;
                 const float wrow = sm.wc[tf & 1][row];
-                const float apart = last_chunks_packed<NG4, NCH4_B, true, O1>(p, tP + tlane, 0, wrow, qr.st, swrite, sidx, lane, &sm.bar_drain);
+                const float apart = last_chunks_packed<NG4, NCH4_B, true, O1>(p, sm.bias[2], sm.wa, tP + tlane, 0, wrow, qr.st, swrite, sidx, lane, &sm.bar_drain);
                 TB(11);
                 if (!DEFER) {
                     if (!finish_sigma(tf, apart, wrow, qr.st, swrite, sidx)) { ok = false; break; }
@@ -1236,8 +1279,9 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
                     pd_apart = apart; pd_wrow = wrow; pd_st = qr.st; pd_sw = swrite; pd_sidx = sidx;
                 }
             }
+            if (tile < 0) break;
         }
-        if (DEFER && ok && my_tiles > 0) finish_sigma(my_tiles - 1, pd_apart, pd_wrow, pd_st, pd_sw, pd_sidx);
+        if (DEFER && ok && t > 0) finish_sigma(t - 1, pd_apart, pd_wrow, pd_st, pd_sw, pd_sidx);
     } else {
         // ============================================================ epilogue warps
         const int quad = warp & 3, grp = warp >> 2;
@@ -1255,7 +1299,7 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
             if constexpr (DEFER) {
 #pragma unroll
                 for (int i = decltype(first)::value; i < decltype(first)::value + decltype(count)::value; ++i)
-                    last_chunk_from_regs<O1>(p, 16 * (1 + grp + NG4 * i), hv[i], d_wrow, d_st, d_sw, d_sidx, lane, d_apart);
+                    last_chunk_from_regs<O1>(p, sm.bias[2], sm.wa, 16 * (1 + grp + NG4 * i), hv[i], d_wrow, d_st, d_sw, d_sidx, lane, d_apart);
             }
         };
         auto held_done = [&](int tf) -> bool {             // the held tile is finished: publish this warp's alpha partial sum
@@ -1268,14 +1312,16 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
         };
         static_assert(!DEFER || NCH4_E == 5, "the deferred schedules split 5 held chunks");
         constexpr int GA = SCHED == 0 ? 2 : SCHED == 1 ? 1 : 0, GB = 2, GC = SCHED == 2 ? 2 : 1, GD = 5 - GA - GB - GC;
-        using I0 = std::integral_constant<int, 0>; using I5 = std::integral_constant<int, 5>;
+        using I0 = std::integral_constant<int, 0>;
         using NA = std::integral_constant<int, GA>; using NB_ = std::integral_constant<int, GB>; using NC = std::integral_constant<int, GC>;
-        using ND = std::integral_constant<int, GD>;
+        using ND = std::integral_constant<int, GD>; using NR = std::integral_constant<int, 5 - GA>;
         using FB = std::integral_constant<int, GA>; using FC = std::integral_constant<int, GA + GB>; using FD = std::integral_constant<int, GA + GB + GC>;
-        for (int t = 0; t < my_tiles && ok; ++t) {
+        int t = 0;
+        for (; ok; ++t) {
             if (DEFER && t > 0 && GA > 0) { held(I0{}, NA{}); TB(21); }          // gap A: the layer-1 MMAs of this tile are running
             // ---- layer 1: accumulator + pre[point of this row] (the hoisted 224 inputs and the bias)
             if (!TW(13, mbar_wait(&sm.bar_prow[t & 1], (uint32_t)(t >> 1) & 1u, p.err, 102))) { ok = false; break; }
+            if (sm.tile_slot[t & 1] < 0) break;                  // no tile left
             Tc8Pf<COOP, PFN> pfs;
             pfs.init(p.pre, &sm.prow[t & 1][quad * 32], lane);
             pfs.prefetch(grp);                                   // in flight under the wait for the layer-1 MMAs
@@ -1293,7 +1339,7 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
                 }
                 if (!TW(16, mbar_wait(&sm.bar_acc_full, n_acc & 1u, p.err, 98))) { ok = false; break; }
                 tc_fence_after();
-                tc8_epi_layer<false, COOP>(sm, ((l & 1) ? tP : tQ) + tlane, grp, p.bias[l], pfs, nullptr);
+                tc8_epi_layer<false, COOP>(sm, ((l & 1) ? tP : tQ) + tlane, grp, sm.bias[l - 1], pfs, nullptr);
                 TB(17);
             }
             if (!ok) break;
@@ -1308,7 +1354,7 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
                 const QuadRow qr = quad_row(sm.qhead[t & 1][quad], (int)sm.qtotal[t & 1][quad], lane);
                 const int sidx = qr.live ? (int)p.vorder[sm.qfirst[t & 1][quad] + qr.j] : 0;
                 if constexpr (!DEFER) {
-                    const float apart = last_chunks_packed<NG4, NCH4_E, true, O1>(p, tP + tlane, 1 + grp, sm.wc[t & 1][erow], qr.st, qr.is_end && sidx < n_valid, sidx,
+                    const float apart = last_chunks_packed<NG4, NCH4_E, true, O1>(p, sm.bias[2], sm.wa, tP + tlane, 1 + grp, sm.wc[t & 1][erow], qr.st, qr.is_end && sidx < n_valid, sidx,
                                                                               lane, &sm.bar_drain);
                     sm.alpha_part[t & 1][grp][erow] = apart;
                     __syncwarp();
@@ -1329,7 +1375,8 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
                 }
             }
         }
-        if (DEFER && ok && my_tiles > 0) { held(I0{}, I5{}); held_done(my_tiles - 1); }
+        if (DEFER && ok && t > 0) { held(FB{}, NR{}); held_done(t - 1); }    // (chunks before FB went in gap A of the end iteration)
+        n_done = t;
     }
     if (prof && tid == 0) prof_add(p, 20, clock64() - _tk0);
 #undef TW
@@ -1338,7 +1385,7 @@ __global__ void __launch_bounds__(DEFER ? tc8::NTHR_DEFER : tc8::NTHR, 1) k_shad
         uint32_t smid;
         asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
         reinterpret_cast<long long*>(p.err)[32 + blockIdx.x] = ((clock64() - _tk0) & 0xffffffffffffll) | ((long long)smid << 48);
-        if (blockIdx.x == 0) reinterpret_cast<long long*>(p.err)[32 + 192] = n_quads;
+        if (blockIdx.x == 0) { reinterpret_cast<long long*>(p.err)[32 + 192] = n_quads; reinterpret_cast<long long*>(p.err)[32 + 193] = n_done; }
     }
     tc_fence_before();
     __syncthreads();
@@ -1689,7 +1736,7 @@ struct TcWs {   // carve-up of the caller's workspace (all sizes from max_valid_
         quad_first = c.take<uint32_t>((size_t)cap + 2);
         vorder = c.take<uint32_t>((size_t)cap + 2);
         vcntp = c.take<unsigned char>((size_t)cap + 16);
-        pack_cnt = c.take<int>(4);
+        pack_cnt = c.take<int>(4);                                    // [0] n_quads, [1] tile queue of k_shade_tc8
     }
 };
 }  // namespace
@@ -1753,6 +1800,7 @@ extern "C" int pnb_shade_forward_tc(const pnb_query_t* q, const pnb_points_t* pt
     p.dbg_no_weights = (flags & PNB_TC_DBG_NO_WEIGHTS) ? 1 : 0;
     p.dbg_flags = (flags >> 8) & 0xff;
     p.vcnt = w.vcntp; p.vorder = w.vorder; p.quad_first = w.quad_first; p.pack_cnt = w.pack_cnt;
+    p.tile_ctr = w.pack_cnt + 1;
     p.pre = d_point_pre;
     p.hbar_fmt = 1;                                           // h-bar in the colour kernel's operand format
     if (flags & PNB_TC_PAIRS) {

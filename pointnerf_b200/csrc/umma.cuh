@@ -349,13 +349,15 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
     hi = __float2bfloat16_rn(x);
     lo = __float2bfloat16_rn(x - __bfloat162float(hi));
 }
-// two floats -> packed hi pair / lo pair (element 0 in the low half)
+// two floats -> packed hi pair / lo pair (element 0 in the low half).  The hi pair is widened back to fp32 with a shift and a mask
+// (exact: a bf16 is the upper half of its fp32): F2FP.PACK_AB + SHF/LOP3 + 2 FADD + F2FP.PACK_AB, without the PRMT extract / re-pack
+// that __low2float / __high2float compile to.
 __device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t& hi, uint32_t& lo) {
-    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-    float ra = a - __low2float(h), rb = b - __high2float(h);
-    __nv_bfloat162 l = __floats2bfloat162_rn(ra, rb);
-    hi = *reinterpret_cast<uint32_t*>(&h);
-    lo = *reinterpret_cast<uint32_t*>(&l);
+    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    hi = *reinterpret_cast<const uint32_t*>(&h);
+    const float ra = a - __uint_as_float(hi << 16), rb = b - __uint_as_float(hi & 0xffff0000u);
+    const __nv_bfloat162 l = __floats2bfloat162_rn(ra, rb);
+    lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 
 }  // namespace umma

@@ -1,6 +1,6 @@
 """Run on the GPU box, lego_render frame: per-CTA cycle counts of the pair kernel (dbg flag 4: cycles + SM id of every CTA into
 d_err[64..]) and the cycles per 128-row tile they imply.  PNB_FROZEN=0 selects the general kernel (k_shade_tc7), default the
-frozen-cloud kernel (k_shade_tc8); PNB_NO_WEIGHTS=1 removes the weight traffic (garbage results, timing experiment);
+frozen-cloud kernel (k_shade_tc8; PNB_DBG_FLAGS=16: static tile schedule instead of the tile queue); PNB_NO_WEIGHTS=1 removes the weight traffic (garbage results, timing experiment);
 PNB_SR / PNB_CONFIG override the workload."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -49,7 +49,7 @@ if os.environ.get("PNB_PROF") and net.frozen_ok:
              "epi warp 0: wait prow", "epi warp 0: wait acc_full (E1)", "epi warp 0: E1 busy", "epi warp 0: wait acc_full (E2,E3)", "epi warp 0: E2+E3 busy",
              "epi warp 0: wait final", "epi warp 0: last-epilogue share (DEFER: drain only)", "kernel total (thread 0)",
              "epi warp 0: deferred last-epilogue chunks (gaps A-C of the next tile)"]
-    tiles0 = (n_tiles - 1) // 148 + 1
+    tiles0 = int(net._err.cpu().view(torch.int64)[32 + 193]) or (n_tiles - 1) // 148 + 1     # tiles block 0 processed (k_shade_tc8)
     print("block 0 accounting (%d tiles), cycles per tile:" % tiles0)
     for n, v in zip(names, c):
         print("  %-46s %9.0f  (%5.1f %% of the kernel)" % (n, v / tiles0, 100.0 * v / max(c[20], 1)))
