@@ -26,6 +26,8 @@
  *                         (fill_invalid: results are written at full R).
  *   pnb_shade_backward / pnb_composite_backward: the autograd of the above (loss.backward() in
  *                         models/mvs_points_volumetric_model.py:98-118).
+ *   pnb_probe_maps / pnb_probe_select: the probe pass of point growing (run/train_ft.py:417-530 with
+ *                         models/neural_points_volumetric_model.py:331-351), one call each per frame.
  */
 #ifndef PNB200_H
 #define PNB200_H
@@ -189,6 +191,31 @@ int pnb_aux_outputs(const pnb_query_t* q, const pnb_points_t* pts, const long lo
  * straight-through estimator, every entry adds its gradient to the conf of its (clamped-to-0) point index. */
 int pnb_aux_conf_backward(const pnb_query_t* q, const long long* d_rows, int n_rows,
                           const float* d_grad_conf_coefficient, float* d_grad_conf, pnb_stream_t stream);
+
+/* ---- point growing: probe outputs and hole selection (run/train_ft.py:417-530) ----
+ * pnb_probe_maps: the probe outputs of models/neural_points_volumetric_model.py:331-351 followed by fill_invalid / unmask (:87-123),
+ * for all R rays of a query, from the compacted query and the [R,SR] opacity of pnb_composite_forward (no dense export).  Per hit ray:
+ * j* = arg-max opacity over the SR slots (first index on ties), op_max [R] = opacity[j*], loc [R,3] = world position of slot j*
+ * (origin for an unfilled slot), far_dist [R] = min over the K slots of |xyz[max(pidx,0)] - loc|, and avg_{color [R,3], dir [R,3],
+ * conf [R], emb [R,32]} = sum over k of attr[max(pidx_k,0)] * w_k * clamp(conf, 1e-4, 1) with the normalised inverse-distance weights.
+ * Rays without a neighbour get zeros.  d_argmax [R] (optional, may be NULL): j*, -1 for rays without a neighbour. */
+int pnb_probe_maps(const pnb_query_t* q, const pnb_points_t* pts, const float* d_opacity, float* d_op_max, float* d_loc,
+                   float* d_far_dist, float* d_avg_color, float* d_avg_dir, float* d_avg_conf, float* d_avg_emb, int32_t* d_argmax,
+                   pnb_stream_t stream);
+/* pnb_probe_select: the hole test of run/train_ft.py:493-512 on an H x W frame, maps in row-major [H*W] layout as probe_hole builds
+ * them (ray_mask int8, 0 where no ray was cast; d_present uint8 = the pixels given (edge_mask), NULL = all; d_gt [H*W,3], 0 where
+ * not given).  A pixel is selected when ray_mask > 0, op_max > opacity_thresh, and either a given pixel with ray_mask < 1 and
+ * |gt - bg| > 0.002 lies in its 3x3 window (clipped to the image), or far_thresh > 0, far_dist > far_thresh and |gt - color| < 0.1.
+ * The selected pixels are compacted in row-major order: the first min(n, cap) go to add_xyz [cap,3] (from d_loc),
+ * add_emb [cap,32], add_color [cap,3], add_dir [cap,3], add_conf [cap]; d_count (device int32) receives n.  Deterministic.
+ * ws >= pnb_probe_select_bytes(H, W); the embedding buffers must be 16-byte aligned. */
+size_t pnb_probe_select_bytes(int H, int W);
+int pnb_probe_select(int H, int W, const int8_t* d_ray_mask, const uint8_t* d_present, const float* d_gt, const float* d_color,
+                     const float* d_far_dist, const float* d_op_max, const float* d_loc, const float* d_avg_emb,
+                     const float* d_avg_color, const float* d_avg_dir, const float* d_avg_conf, const float bg_color[3],
+                     float opacity_thresh, float far_thresh, void* ws, size_t ws_bytes, int cap, float* d_add_xyz,
+                     float* d_add_emb, float* d_add_color, float* d_add_dir, float* d_add_conf, int32_t* d_count,
+                     pnb_stream_t stream);
 
 /* ---- shading forward on the tensor cores (tcgen05 / TMEM, BF16x3 error-compensated split) ---- */
 /* Packs block1 / block3 / colour-branch weights of a pnb_mlp_t (fp32 W^T buffers) into tcgen05 operand images (hi/lo bf16, UMMA

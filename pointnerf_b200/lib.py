@@ -58,7 +58,8 @@ QC = dict(n_cand=0, n_valid=1, n_pairs=2, R1=3, R2=4, overflow=5)
 SYMBOLS = ["pnb_version", "pnb_last_error", "pnb_struct_size", "pnb_grid_bytes", "pnb_grid_build", "pnb_query_bytes", "pnb_query",
            "pnb_query_export", "pnb_shade_bytes", "pnb_shade_forward", "pnb_composite_forward",
            "pnb_mlp_pack_bytes", "pnb_mlp_pack", "pnb_point_pre_bytes", "pnb_point_pre", "pnb_shade_tc_bytes", "pnb_shade_forward_tc",
-           "pnb_shade_tc_tables", "pnb_backward_bytes", "pnb_shade_backward", "pnb_aux_outputs", "pnb_aux_conf_backward"]
+           "pnb_shade_tc_tables", "pnb_backward_bytes", "pnb_shade_backward", "pnb_aux_outputs", "pnb_aux_conf_backward",
+           "pnb_probe_maps", "pnb_probe_select_bytes", "pnb_probe_select"]
 # test-only library (csrc/selftest/pnb200_selftest.h)
 SELFTEST_LIB_PATH = os.path.join(_HERE, "csrc", "libpnb200_selftest.so")
 SELFTEST_SYMBOLS = ["pnb_selftest_last_error", "pnb_umma_selftest", "pnb_umma_bench", "pnb_umma_selftest2", "pnb_gemm_tc_test"]
@@ -116,6 +117,14 @@ def load():
                                     C.c_void_p, C.c_void_p]
     lib.pnb_aux_conf_backward.restype = C.c_int
     lib.pnb_aux_conf_backward.argtypes = [C.POINTER(Query), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.pnb_probe_maps.restype = C.c_int
+    lib.pnb_probe_maps.argtypes = [C.POINTER(Query), C.POINTER(Points), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.pnb_probe_select_bytes.restype = C.c_size_t
+    lib.pnb_probe_select_bytes.argtypes = [C.c_int, C.c_int]
+    lib.pnb_probe_select.restype = C.c_int
+    lib.pnb_probe_select.argtypes = [C.c_int, C.c_int] + [C.c_void_p] * 11 + [C.POINTER(C.c_float), C.c_float, C.c_float, C.c_void_p,
+                                                                             C.c_size_t, C.c_int] + [C.c_void_p] * 7
     lib.pnb_mlp_pack_bytes.restype = C.c_size_t
     lib.pnb_mlp_pack_bytes.argtypes = []
     lib.pnb_mlp_pack.restype = C.c_int

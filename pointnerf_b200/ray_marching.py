@@ -9,6 +9,8 @@
                          (/root/reference/models/neural_points_volumetric_model.py:252-364)
   render_full(...)       the same computation with full-R outputs (fill_invalid already applied,
                          :87-123) and NO host synchronisation -- what bench.py times.
+  probe_full(...)        render_full + the probe outputs of point growing (:331-351) for all rays, one kernel
+                         (pnb_probe_maps) -- what runner.probe_frame / probe_holes use.
 
 Only the shipped hot-path configuration (SURVEY.md section 8 head) is implemented; any other option
 value raises NotImplementedError (no silent fallback).
@@ -369,7 +371,7 @@ def _init_state(mod):
     mod._pnb_ready = True
 
 
-_PATCHED = ("forward", "_run", "check_errors", "render_full", "_point_pre", "_poll_status", "_queue_status")
+_PATCHED = ("forward", "_run", "check_errors", "render_full", "_point_pre", "_poll_status", "_queue_status", "probe_full")
 
 
 def install_into(reference_cls):
@@ -552,6 +554,36 @@ class NeuralPointsRayMarching(nn.Module):
         self._queue_status(q, ray_color.device)
         return dict(coarse_raycolor=ray_color[None], coarse_point_opacity=opacity[None],
                     coarse_is_background=bg_T[None, :, None], ray_mask=ray_mask[None])
+
+    def probe_full(self, campos, raydir, camrotc2w, near, far, bg_color, t=None, want_argmax=False):
+        """render_full() plus the probe outputs of point growing for all R rays (neural_points_volumetric_model.py:331-351 followed by
+        fill_invalid / unmask, :87-123; one pnb_probe_maps kernel on the compacted query, no dense export, no host sync).  Adds
+        ray_max_shading_opacity [1,R,1], ray_max_sample_loc_w [1,R,3], ray_max_far_dist [1,R,1], shading_avg_color [1,R,3],
+        shading_avg_dir [1,R,3], shading_avg_conf [1,R,1], shading_avg_embedding [1,R,32] (zeros on rays without a neighbour) and,
+        with want_argmax, ray_max_slot [1,R] int32 (the arg-max sample slot, -1 without a neighbour).  Status as render_full."""
+        q, ray_color, opacity, bg_T, ray_mask = self._run(campos, raydir, camrotc2w, near, far, bg_color, False, t=t, frozen=True)
+        dev = ray_color.device
+        R = q.R
+        # one allocation carved into contiguous maps; the embedding block comes first (16-byte aligned rows for pnb_probe_select)
+        flat = torch.empty((R * 44,), dtype=torch.float32, device=dev)
+        emb = flat[:R * 32].view(R, 32)
+        loc, col, pdir = (flat[R * o:R * (o + 3)].view(R, 3) for o in (32, 35, 38))
+        op_max, far_d, conf = (flat[R * o:R * (o + 1)].view(R, 1) for o in (41, 42, 43))
+        argmax = torch.empty((R,), dtype=torch.int32, device=dev) if want_argmax else None
+        lib = _lib.load()
+        pts = points_desc_of(self.neural_points)
+        _lib.check(lib.pnb_probe_maps(_lib.C.byref(q.desc), _lib.C.byref(pts), opacity.data_ptr(), op_max.data_ptr(), loc.data_ptr(),
+                                      far_d.data_ptr(), col.data_ptr(), pdir.data_ptr(), conf.data_ptr(), emb.data_ptr(),
+                                      argmax.data_ptr() if argmax is not None else None,
+                                      torch.cuda.current_stream(dev).cuda_stream), "pnb_probe_maps")
+        self._queue_status(q, dev)
+        out = dict(coarse_raycolor=ray_color[None], coarse_point_opacity=opacity[None], coarse_is_background=bg_T[None, :, None],
+                   ray_mask=ray_mask[None], ray_max_shading_opacity=op_max[None], ray_max_sample_loc_w=loc[None],
+                   ray_max_far_dist=far_d[None], shading_avg_color=col[None], shading_avg_dir=pdir[None], shading_avg_conf=conf[None],
+                   shading_avg_embedding=emb[None])
+        if argmax is not None:
+            out["ray_max_slot"] = argmax[None]
+        return out
 
     def forward(self, campos, raydir, gt_image=None, bg_color=None, camrotc2w=None, pixel_idx=None, near=None,
                 far=None, focal=None, h=None, w=None, intrinsic=None, **kargs):
