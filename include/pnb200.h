@@ -61,7 +61,18 @@ enum {
     PNB_GC_OVERFLOW_P = 3, /* some voxel > P (reference: random reservoir; here: first P by index, flagged) */
     PNB_GC_N_INRANGE = 4,  /* points inside the grid */
     PNB_GC_SLOT0_CELL = 5, /* linear index of the voxel that holds the lowest-index in-range point (Q1) */
-    PNB_GC_FIRST_PT = 6    /* that point's index */
+    PNB_GC_FIRST_PT = 6,   /* that point's index */
+    /* bounding box of the dilated occupancy (occ_bits), inclusive voxel coordinates; empty (lo > hi) when no point is in range.
+     * pnb_query marches only the steps of a ray that can reach it (a wider box is always safe, a narrower one is not). */
+    PNB_GC_BOX_X0 = 7,
+    PNB_GC_BOX_Y0 = 8,
+    PNB_GC_BOX_Z0 = 9,
+    PNB_GC_BOX_X1 = 10,
+    PNB_GC_BOX_Y1 = 11,
+    PNB_GC_BOX_Z1 = 12,
+    /* squared radius (fp32 bits) of a sphere about the grid centre lo + dim * svs / 2 that holds every voxel of occ_bits; the march
+     * also skips the steps outside it */
+    PNB_GC_SPHERE_R2 = 13
 };
 
 /* counters written by pnb_query (device int32[16]) */
@@ -157,7 +168,8 @@ int pnb_grid_build(pnb_grid_t* grid, void* buf, size_t buf_bytes, const float* d
 
 /* ---- query ---- */
 size_t pnb_query_bytes(int R, int SR, int K, int cap_samples);
-/* cap_samples <= 0 -> R*SR (can never overflow).  t: [D] (t_ray_stride 0) or [R,D] (t_ray_stride D). */
+/* cap_samples <= 0 -> R*SR (can never overflow).  t: [D] (t_ray_stride 0) or [R,D] (t_ray_stride D), every row non-decreasing
+ * (as near-far linear ray generation makes it: the march finds the steps inside the grid's occupied box by binary search). */
 int pnb_query(pnb_query_t* q, void* ws, size_t ws_bytes, const pnb_grid_t* grid, const float campos[3],
               const float* d_raydir, int R, const float* d_t, int t_ray_stride, int D, int SR, int K,
               float radius_limit, const int32_t kernel_size[3], int cap_samples, pnb_stream_t stream,

@@ -78,6 +78,8 @@ __device__ __forceinline__ int vox1(float p, float lo, float svs) {
 __device__ __forceinline__ float raypos1(float c, float dir, float t) {
     return __fadd_rn(c, __fmul_rn(dir, t));
 }
+// Centre of the grid along axis a: the centre of the bounding sphere PNB_GC_SPHERE_R2.
+__device__ __forceinline__ float grid_centre(float lo, float svs, int dim) { return lo + 0.5f * (float)dim * svs; }
 __device__ __forceinline__ bool in_grid(int x, int y, int z, const int* dim) {
     return (x >= 0) & (x < dim[0]) & (y >= 0) & (y < dim[1]) & (z >= 0) & (z < dim[2]);
 }

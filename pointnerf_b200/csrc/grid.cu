@@ -142,6 +142,27 @@ __global__ void __launch_bounds__(256) k_mark(const float* __restrict__ xyz, Bui
     atomicOr(&pt_bits[c >> 5], 1u << (c & 31));
     atomicMin(&counters[PNB_GC_FIRST_PT], i);
     atomicAdd(&counters[PNB_GC_N_INRANGE], 1);
+    // Squared distance from the grid centre to the farthest corner of the voxels that k_dilate marks around this point: the
+    // farthest point of an axis-aligned box from a centre is the corner that is farthest along every axis.
+    const int vv[3] = {x, y, z};
+    float r2 = 0.f;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const float ctr = grid_centre(p.lo[a], p.svs[a], p.dim[a]);
+        const float e0 = p.lo[a] + (float)(vv[a] - p.qs[a] / 2) * p.svs[a], e1 = p.lo[a] + (float)(vv[a] + (p.qs[a] + 1) / 2) * p.svs[a];
+        const float m = fmaxf(fabsf(e0 - ctr), fabsf(e1 - ctr));
+        r2 += m * m;
+    }
+    // box of the voxels holding points (k_finish dilates it) and the sphere; reduced over the warp first, so that the counters see
+    // one atomic per warp and value instead of one per point (r2 >= 0: its bits order as the floats do)
+    const uint32_t act = __activemask();
+    const int r2max = __reduce_max_sync(act, __float_as_int(r2));
+    const int v[6] = {__reduce_min_sync(act, x), __reduce_min_sync(act, y), __reduce_min_sync(act, z),
+                      __reduce_max_sync(act, x), __reduce_max_sync(act, y), __reduce_max_sync(act, z)};
+    if ((threadIdx.x & 31) == __ffs(act) - 1) {
+        for (int a = 0; a < 3; ++a) { atomicMin(&counters[PNB_GC_BOX_X0 + a], v[a]); atomicMax(&counters[PNB_GC_BOX_X1 + a], v[3 + a]); }
+        atomicMax(&counters[PNB_GC_SPHERE_R2], r2max);
+    }
 }
 
 // pass 2: cell -> slot, count points per slot.
@@ -219,10 +240,17 @@ __global__ void __launch_bounds__(256) k_dilate(BuildParams p, uint32_t n_words,
     }
 }
 
-__global__ void k_finish(const uint32_t* word_rank, uint32_t n_words, int max_o, int* counters) {
+__global__ void k_finish(BuildParams p, const uint32_t* word_rank, uint32_t n_words, int max_o, int* counters) {
     int n_occ = (int)word_rank[n_words];
     counters[PNB_GC_N_OCC] = n_occ;
     if (n_occ > max_o) counters[PNB_GC_OVERFLOW_O] = 1;
+    // the point box grown by k_dilate's window: [c - qs/2, c + (qs+1)/2) clipped to the grid (an empty box stays empty)
+    if (n_occ > 0) {
+        for (int a = 0; a < 3; ++a) {
+            counters[PNB_GC_BOX_X0 + a] = max(0, counters[PNB_GC_BOX_X0 + a] - p.qs[a] / 2);
+            counters[PNB_GC_BOX_X1 + a] = min(p.dim[a] - 1, counters[PNB_GC_BOX_X1 + a] + (p.qs[a] + 1) / 2 - 1);
+        }
+    }
 }
 
 struct GridLayout {
@@ -300,13 +328,14 @@ extern "C" int pnb_grid_build(pnb_grid_t* grid, void* buf, size_t buf_bytes, con
     for (int i = 0; i < 16; ++i) init[i] = 0;
     init[PNB_GC_FIRST_PT] = 0x7fffffff;
     init[PNB_GC_SLOT0_CELL] = -1;
+    for (int a = 0; a < 3; ++a) { init[PNB_GC_BOX_X0 + a] = 0x7fffffff; init[PNB_GC_BOX_X1 + a] = -1; }
     PNB_CHECK_CUDA(cudaMemcpyAsync(L.counters, init, sizeof(init), cudaMemcpyHostToDevice, stream));
 
     int nbN = (N + 255) / 256;
     k_mark<<<nbN, 256, 0, stream>>>(d_xyz, p, L.pt_bits, L.pt_cell, L.counters);
     int rc = exclusive_scan_u32(L.pt_bits, 1, L.word_rank, nw, L.scan_tmp, stream);
     if (rc) return rc;
-    k_finish<<<1, 1, 0, stream>>>(L.word_rank, nw, max_o, L.counters);
+    k_finish<<<1, 1, 0, stream>>>(p, L.word_rank, nw, max_o, L.counters);
     // cell_cnt is accumulated in cell_fill, scanned into cell_start, then cell_fill is re-zeroed as cursor
     k_count<<<nbN, 256, 0, stream>>>(p, L.pt_bits, L.word_rank, L.pt_cell, L.cell_fill, L.counters);
     rc = exclusive_scan_u32(L.cell_fill, 0, L.cell_start, (uint32_t)N, L.scan_tmp, stream);

@@ -27,7 +27,42 @@ struct QueryParams {
     int cap;
 };
 
+// First index d of the non-decreasing row tr[0, D) with tr[d] >= v (LE = false) or tr[d] > v (LE = true); D if there is none.
+// Warp-cooperative: every round probes 32 evenly spaced entries and keeps the gap where the predicate turns (2 rounds for D = 400).
+template <bool LE>
+__device__ __forceinline__ int warp_search(const float* tr, int D, float v, int lane) {
+    int lo = 0, hi = D;  // the answer lies in [lo, hi]; hi == D or tr[hi] passes
+    while (lo < hi) {
+        const int step = (hi - lo + 31) / 32;
+        const int i = lo + lane * step;
+        bool below = false;
+        if (i < hi) {
+            const float t = tr[i];
+            below = LE ? !(t > v) : (t < v);
+        }
+        const int k = __popc(__ballot_sync(0xffffffffu, below));  // probes 0..k-1 fail, probe k (if any) passes
+        if (k == 0) break;
+        const int last = lo + (k - 1) * step;
+        lo = last + 1;
+        hi = min(hi, last + step);
+    }
+    return lo;
+}
+
 // One warp per ray: 32 march steps per iteration, ballot -> ordered slots.
+//
+// Only the steps that can land in the occupied box (PNB_GC_BOX_*, the bounding box of occ_bits) are marched.  A step hits only if
+// its voxel floor(fdiv(fsub(p, lo), svs)) lies in the box, with p = fadd(c, fmul(d, t)).  Such a p lies within a few ulps of the
+// box's world extent [lo + b0 * svs, lo + (b1 + 1) * svs], and c + d * t (exact) within a few more ulps of p.  The box is widened by
+// one voxel on every side before the ray is clipped, so the clipped t-interval [t0, t1], computed in fp32 with errors of a few ulps
+// of t, still holds every t that can hit as long as a voxel is far wider than those rounding errors (|d| ulp(t) + ulp(p) against
+// svs: 1e-6 against 8e-3 for the shipped scenes).  The steps kept are those from the last one before t0 to the first one after t1,
+// one more step on each side than the interval needs.  Every skipped step is outside the widened box, so it is at least one voxel
+// away from any occupied voxel and its exact per-step test would fail: slots, counts and order are those of the full march.
+// The same holds for the bounding sphere (PNB_GC_SPHERE_R2, about the grid centre): every point of an occupied voxel lies within
+// its radius, which is widened by one voxel before the ray is clipped.  For a rounded object it removes most of the steps of the
+// rays that cross the box's corners without meeting the object.  Setting the box and the radius to cover everything (tests) gives
+// the full march.
 __global__ void __launch_bounds__(256) k_march(QueryParams p, int* __restrict__ nsamp, uint16_t* __restrict__ steps) {
     int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     int lane = threadIdx.x & 31;
@@ -35,41 +70,86 @@ __global__ void __launch_bounds__(256) k_march(QueryParams p, int* __restrict__ 
     const int r = warp;
     const float dx = p.raydir[3 * r], dy = p.raydir[3 * r + 1], dz = p.raydir[3 * r + 2];
     const float* tr = p.t + (size_t)r * p.t_ray_stride;
-    int count = 0;
-    for (int base = 0; base < p.D; base += 32) {
-        int d = base + lane;
-        bool hit = false;
-        if (d < p.D) {
-            float t = tr[d];
-            int x = vox1(raypos1(p.campos[0], dx, t), p.g.lo[0], p.g.svs[0]);
-            int y = vox1(raypos1(p.campos[1], dy, t), p.g.lo[1], p.g.svs[1]);
-            int z = vox1(raypos1(p.campos[2], dz, t), p.g.lo[2], p.g.svs[2]);
-            if (in_grid(x, y, z, p.g.dim)) {
-                uint32_t c = cell_index(x, y, z, p.g.dim);
-                hit = (__ldg(&p.g.occ_bits[c >> 5]) >> (c & 31)) & 1u;
-            }
+    // clip the ray to the widened box
+    const float c3[3] = {p.campos[0], p.campos[1], p.campos[2]}, d3[3] = {dx, dy, dz};
+    float t0 = -INFINITY, t1 = INFINITY;
+    bool miss = false;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const int b0 = __ldg(&p.g.counters[PNB_GC_BOX_X0 + a]), b1 = __ldg(&p.g.counters[PNB_GC_BOX_X1 + a]);
+        const float wlo = p.g.lo[a] + (float)(b0 - 1) * p.g.svs[a], whi = p.g.lo[a] + (float)(b1 + 2) * p.g.svs[a];
+        miss |= b0 > b1;
+        if (d3[a] != 0.f) {
+            const float ta = (wlo - c3[a]) / d3[a], tb = (whi - c3[a]) / d3[a];
+            t0 = fmaxf(t0, fminf(ta, tb));
+            t1 = fminf(t1, fmaxf(ta, tb));
+        } else {
+            miss |= c3[a] < wlo || c3[a] > whi;
         }
-        uint32_t m = __ballot_sync(0xffffffffu, hit);
-        int slot = count + __popc(m & ((1u << lane) - 1u));
-        if (hit && slot < p.SR) steps[(size_t)r * p.SR + slot] = (uint16_t)d;
-        count += __popc(m);
-        if (count >= p.SR) break;
+    }
+    // and to the bounding sphere, widened by one voxel; |d|^2 t^2 + 2 (d . oc) t + |oc|^2 - rad^2 = 0
+    {
+        float oc[3], a2 = 0.f, b = 0.f, k = 0.f, svs_max = 0.f;
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            oc[a] = c3[a] - grid_centre(p.g.lo[a], p.g.svs[a], p.g.dim[a]);
+            a2 += d3[a] * d3[a]; b += d3[a] * oc[a]; k += oc[a] * oc[a];
+            svs_max = fmaxf(svs_max, p.g.svs[a]);
+        }
+        const float rad = sqrtf(__int_as_float(__ldg(&p.g.counters[PNB_GC_SPHERE_R2]))) + svs_max;
+        const float disc = b * b - a2 * (k - rad * rad);
+        if (disc >= 0.f && a2 > 0.f) {
+            const float sq = sqrtf(disc);
+            t0 = fmaxf(t0, (-b - sq) / a2);
+            t1 = fminf(t1, (-b + sq) / a2);
+        } else {
+            miss = true;
+        }
+    }
+    miss |= !(t0 <= t1);
+    int count = 0;
+    if (!miss) {
+        const int first = max(warp_search<false>(tr, p.D, t0, lane) - 1, 0);   // first step with t >= t0, one step earlier
+        const int end = min(warp_search<true>(tr, p.D, t1, lane) + 1, p.D);    // past the last step with t <= t1, one step later
+        for (int base = first; base < end; base += 32) {
+            int d = base + lane;
+            bool hit = false;
+            if (d < end) {
+                float t = tr[d];
+                int x = vox1(raypos1(p.campos[0], dx, t), p.g.lo[0], p.g.svs[0]);
+                int y = vox1(raypos1(p.campos[1], dy, t), p.g.lo[1], p.g.svs[1]);
+                int z = vox1(raypos1(p.campos[2], dz, t), p.g.lo[2], p.g.svs[2]);
+                if (in_grid(x, y, z, p.g.dim)) {
+                    uint32_t c = cell_index(x, y, z, p.g.dim);
+                    hit = (__ldg(&p.g.occ_bits[c >> 5]) >> (c & 31)) & 1u;
+                }
+            }
+            uint32_t m = __ballot_sync(0xffffffffu, hit);
+            int slot = count + __popc(m & ((1u << lane) - 1u));
+            if (hit && slot < p.SR) steps[(size_t)r * p.SR + slot] = (uint16_t)d;
+            count += __popc(m);
+            if (count >= p.SR) break;
+        }
     }
     if (lane == 0) nsamp[r] = count < p.SR ? count : p.SR;
 }
 
-// candidate s -> packed (ray, slot)
-__global__ void __launch_bounds__(256) k_expand(int R, int SR, int cap, const int* __restrict__ nsamp,
-                                                const uint32_t* __restrict__ samp_off, uint32_t* __restrict__ samp_ray,
-                                                int* counters) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= R * SR) return;
-    int r = i / SR, j = i - r * SR;
-    if (j >= nsamp[r]) return;
-    uint32_t s = samp_off[r] + j;
-    if (s >= (uint32_t)cap) { counters[PNB_QC_OVERFLOW] = 1; return; }
-    samp_ray[s] = ((uint32_t)r << 7) | (uint32_t)j;
-    if (j == 0) atomicAdd(&counters[PNB_QC_R1], 1);
+// candidates of ray r -> packed (ray, slot); one thread per ray
+__global__ void __launch_bounds__(256) k_expand(int R, int cap, const int* __restrict__ nsamp, const uint32_t* __restrict__ samp_off,
+                                                uint32_t* __restrict__ samp_ray, int* counters) {
+    int r = blockIdx.x * blockDim.x + threadIdx.x;
+    bool first = false;
+    if (r < R) {
+        const int n = nsamp[r];
+        const uint32_t off = samp_off[r];
+        first = n > 0 && off < (uint32_t)cap;
+        for (int j = 0; j < n; ++j) {
+            if (off + j >= (uint32_t)cap) { counters[PNB_QC_OVERFLOW] = 1; break; }
+            samp_ray[off + j] = ((uint32_t)r << 7) | (uint32_t)j;
+        }
+    }
+    const uint32_t m = __ballot_sync(0xffffffffu, first);
+    if ((threadIdx.x & 31) == 0 && m) atomicAdd(&counters[PNB_QC_R1], __popc(m));
 }
 
 // One thread per candidate sample: canonical layered K-NN.
@@ -104,40 +184,58 @@ __global__ void __launch_bounds__(128) k_knn(QueryParams p, const uint32_t* __re
         const int ya = max(-fy, -layer), yb = min(p.g.dim[1] - fy, layer + 1);
         const int za = max(-fz, -layer), zb = min(p.g.dim[2] - fz, layer + 1);
         for (int x = xa; x < xb; ++x)
-            for (int y = ya; y < yb; ++y)
-                for (int z = za; z < zb; ++z) {
-                    if (max(abs(z), max(abs(x), abs(y))) != layer) continue;
-                    uint32_t c = cell_index(fx + x, fy + y, fz + z, p.g.dim);
-                    uint32_t w = __ldg(&p.g.pt_bits[c >> 5]);
-                    if (!((w >> (c & 31)) & 1u)) continue;
-                    if ((int)c == dead) continue;  // query_worldcoords.cu:147 (slot 0 never filled)
-                    uint32_t slot = __ldg(&p.g.word_rank[c >> 5]) + __popc(w & ((1u << (c & 31)) - 1u));
-                    uint32_t a = __ldg(&p.g.cell_start[slot]), b = __ldg(&p.g.cell_start[slot + 1]);
-                    if (b - a > (uint32_t)p.g.P) b = a + (uint32_t)p.g.P;
-                    for (uint32_t g = a; g < b; ++g) {
-                        float4 q = __ldg(&p.g.spts[g]);
-                        float xv = __fsub_rn(q.x, cx), yv = __fsub_rn(q.y, cy), zv = __fsub_rn(q.z, cz);
-                        float d2 = __fmaf_rn(zv, zv, __fmaf_rn(xv, xv, __fmul_rn(yv, yv)));
-                        if (p.r2 == 0.f || d2 <= p.r2) {
-                            int pi = __float_as_int(q.w);
-                            if (kid++ < p.K) {
-                                int slotk = kid - 1;
+            for (int y = ya; y < yb; ++y) {
+                // The shell cells of column (x, y) are consecutive in z, so they are looked up together: one or two pt_bits words
+                // give their occupancy, one word_rank load their consecutive dense slots, and their cell_start entries share a line.
+                // On the shell's rim every z of [za, zb) is visited, inside it only z = -layer and z = +layer.
+                const bool rim = max(abs(x), abs(y)) == layer;
+                for (int zc = za; zc < zb; zc += 32) {
+                    const int n = min(zb - zc, 32);  // cells zc .. zc + n - 1
+                    const uint32_t span = n == 32 ? 0xffffffffu : (1u << n) - 1u;
+                    const uint32_t want = rim ? span : ((zc == -layer ? 1u : 0u) | (zc + n == layer + 1 ? 1u << (n - 1) : 0u));
+                    if (!want) continue;
+                    const uint32_t c0 = cell_index(fx + x, fy + y, fz + zc, p.g.dim);
+                    const uint32_t wi = c0 >> 5, sh = c0 & 31u;
+                    uint64_t W = __ldg(&p.g.pt_bits[wi]);
+                    if (sh + (uint32_t)n > 32u) W |= (uint64_t)__ldg(&p.g.pt_bits[wi + 1]) << 32;  // the column straddles two words
+                    const uint32_t occ = (uint32_t)(W >> sh) & span;                              // bit i: cell c0 + i holds points
+                    uint32_t todo = occ & want;
+                    if (!todo) continue;
+                    // word_rank[wi + 1] = word_rank[wi] + popc(pt_bits[wi]): one rank serves both words
+                    const uint32_t slot0 = __ldg(&p.g.word_rank[wi]) + __popcll(W & ((1ull << sh) - 1ull));
+                    while (todo) {
+                        const int i = __ffs(todo) - 1;
+                        todo &= todo - 1u;
+                        if ((int)(c0 + i) == dead) continue;  // query_worldcoords.cu:147 (slot 0 never filled)
+                        const uint32_t slot = slot0 + __popc(occ & ((1u << i) - 1u));
+                        uint32_t a = __ldg(&p.g.cell_start[slot]), b = __ldg(&p.g.cell_start[slot + 1]);
+                        if (b - a > (uint32_t)p.g.P) b = a + (uint32_t)p.g.P;
+                        for (uint32_t g = a; g < b; ++g) {
+                            float4 q = __ldg(&p.g.spts[g]);
+                            float xv = __fsub_rn(q.x, cx), yv = __fsub_rn(q.y, cy), zv = __fsub_rn(q.z, cz);
+                            float d2 = __fmaf_rn(zv, zv, __fmaf_rn(xv, xv, __fmul_rn(yv, yv)));
+                            if (p.r2 == 0.f || d2 <= p.r2) {
+                                int pi = __float_as_int(q.w);
+                                if (kid++ < p.K) {
+                                    int slotk = kid - 1;
 #pragma unroll
-                                for (int m = 0; m < PNB_MAX_K; ++m)
-                                    if (m == slotk) { idx[m] = pi; buf[m] = d2; }
-                                if (d2 > far2) { far2 = d2; far_ind = slotk; }
-                            } else if (d2 < far2) {
+                                    for (int m = 0; m < PNB_MAX_K; ++m)
+                                        if (m == slotk) { idx[m] = pi; buf[m] = d2; }
+                                    if (d2 > far2) { far2 = d2; far_ind = slotk; }
+                                } else if (d2 < far2) {
 #pragma unroll
-                                for (int m = 0; m < PNB_MAX_K; ++m)
-                                    if (m == far_ind) { idx[m] = pi; buf[m] = d2; }
-                                far2 = d2;
+                                    for (int m = 0; m < PNB_MAX_K; ++m)
+                                        if (m == far_ind) { idx[m] = pi; buf[m] = d2; }
+                                    far2 = d2;
 #pragma unroll
-                                for (int m = 0; m < PNB_MAX_K; ++m)
-                                    if (m < p.K && buf[m] > far2) { far2 = buf[m]; far_ind = m; }
+                                    for (int m = 0; m < PNB_MAX_K; ++m)
+                                        if (m < p.K && buf[m] > far2) { far2 = buf[m]; far_ind = m; }
+                                }
                             }
                         }
                     }
                 }
+            }
         if (kid >= p.K) break;
     }
     int nv = kid < p.K ? kid : p.K;
@@ -295,7 +393,7 @@ extern "C" int pnb_query(pnb_query_t* q, void* ws, size_t ws_bytes, const pnb_gr
     int rc;
     rc = exclusive_scan_u32(L.nsamp, 3, L.samp_off, (uint32_t)R, L.scan_tmp, stream);
     if (rc) return rc;
-    k_expand<<<(R * SR + 255) / 256, 256, 0, stream>>>(R, SR, cap, L.nsamp, L.samp_off, L.samp_ray, L.counters);
+    k_expand<<<(R + 255) / 256, 256, 0, stream>>>(R, cap, L.nsamp, L.samp_off, L.samp_ray, L.counters);
     k_knn<<<(cap + 127) / 128, 128, 0, stream>>>(p, L.samp_off, L.samp_ray, L.steps, L.cand_pidx, L.samp_nvalid,
                                                   L.ray_hit, L.counters);
     PNB_CHECK_CUDA(cudaGetLastError());

@@ -1440,6 +1440,9 @@ struct Smem {
     unsigned char pe[2][BLK];                // PE(view) K block, hi/lo
     unsigned char b[NSTAGE][2][BLK];         // weight ring: hi / lo image of one K block
     float part[128][4];
+    float4 w3[128];                          // colour_branch.6 W^T rows (x, y, z, 0)
+    float bias[3][128];                      // colour_branch.{0,2,4} biases
+    float b3[4];
     uint64_t bar_full[NSTAGE], bar_empty[NSTAGE], bar_a_full, bar_a_free, bar_pe_ready, bar_acc_full, bar_drain, bar_kblk[4];
     uint32_t tmem_base;
 };
@@ -1468,6 +1471,10 @@ __global__ void __launch_bounds__(ctc2::NTHR, 1) k_color_tc2(ColorTcParams p) {
         mbar_fence_init();
     }
     if (warp == W_ISSUE) tmem_alloc<512>(&sm.tmem_base);
+    // the epilogue's small parameters, read as warp-broadcast shared loads
+    for (int i = tid; i < 3 * 128; i += NTHR) sm.bias[i >> 7][i & 127] = __ldg(p.bias[i >> 7] + (i & 127));
+    for (int i = tid; i < 128; i += NTHR) sm.w3[i] = make_float4(__ldg(p.w3t + 3 * i), __ldg(p.w3t + 3 * i + 1), __ldg(p.w3t + 3 * i + 2), 0.f);
+    if (tid < 3) sm.b3[tid] = __ldg(p.b3 + tid);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -1612,7 +1619,7 @@ __global__ void __launch_bounds__(ctc2::NTHR, 1) k_color_tc2(ColorTcParams p) {
                 if (!mbar_wait(&sm.bar_acc_full, n_acc & 1u, p.err, 90)) { ok = false; break; }
                 tc_fence_after();
                 const uint32_t accb = ((l == 1) ? tY : tX) + tlane;
-                const float* bias = p.bias[l];
+                const float* bias = sm.bias[l];
                 if (l < 2) {
 #pragma unroll
                     for (int i = 0; i < NCH; ++i) {
@@ -1623,7 +1630,7 @@ __global__ void __launch_bounds__(ctc2::NTHR, 1) k_color_tc2(ColorTcParams p) {
                         uint32_t hh[8], ll[8];
 #pragma unroll
                         for (int e = 0; e < 8; ++e) {
-                            float2 bb = __ldg(reinterpret_cast<const float2*>(bias + c0) + e);
+                            float2 bb = reinterpret_cast<const float2*>(bias + c0)[e];
                             float y0 = __uint_as_float(v[2 * e]) + bb.x, y1 = __uint_as_float(v[2 * e + 1]) + bb.y;
                             y0 = fmaxf(y0, tc::LEAKY * y0); y1 = fmaxf(y1, tc::LEAKY * y1);
                             split_bf16x2(y0, y1, hh[e], ll[e]);
@@ -1645,10 +1652,10 @@ __global__ void __launch_bounds__(ctc2::NTHR, 1) k_color_tc2(ColorTcParams p) {
                         tmem_ld_wait();
 #pragma unroll
                         for (int e = 0; e < 16; ++e) {
-                            float y = __uint_as_float(v[e]) + __ldg(bias + c0 + e);
+                            float y = __uint_as_float(v[e]) + bias[c0 + e];
                             y = fmaxf(y, tc::LEAKY * y);
-                            const float* wr = p.w3t + (c0 + e) * 3;
-                            d0 = fmaf(y, __ldg(wr), d0); d1 = fmaf(y, __ldg(wr + 1), d1); d2 = fmaf(y, __ldg(wr + 2), d2);
+                            const float4 wr = sm.w3[c0 + e];
+                            d0 = fmaf(y, wr.x, d0); d1 = fmaf(y, wr.y, d1); d2 = fmaf(y, wr.z, d2);
                         }
                     }
                     tc_fence_before();
@@ -1662,9 +1669,9 @@ __global__ void __launch_bounds__(ctc2::NTHR, 1) k_color_tc2(ColorTcParams p) {
                             const uint32_t s = q.valid_list[vi];
                             float4 o4;
                             o4.x = p.sigma[vi];
-                            const float r0 = d0 + sm.part[erow][0] + __ldg(p.b3);
-                            const float r1 = d1 + sm.part[erow][1] + __ldg(p.b3 + 1);
-                            const float r2 = d2 + sm.part[erow][2] + __ldg(p.b3 + 2);
+                            const float r0 = d0 + sm.part[erow][0] + sm.b3[0];
+                            const float r1 = d1 + sm.part[erow][1] + sm.b3[1];
+                            const float r2 = d2 + sm.part[erow][2] + sm.b3[2];
                             o4.y = 1.0f / (1.0f + expf(-r0)) * (1.0f + 2.0f * 0.001f) - 0.001f;
                             o4.z = 1.0f / (1.0f + expf(-r1)) * (1.0f + 2.0f * 0.001f) - 0.001f;
                             o4.w = 1.0f / (1.0f + expf(-r2)) * (1.0f + 2.0f * 0.001f) - 0.001f;

@@ -51,7 +51,8 @@ class Points(C.Structure):
                 ("conf", C.c_void_p), ("N", C.c_int32)]
 
 
-GC = dict(n_occ=0, max_pts=1, overflow_o=2, overflow_p=3, n_inrange=4, slot0_cell=5, first_pt=6)
+GC = dict(n_occ=0, max_pts=1, overflow_o=2, overflow_p=3, n_inrange=4, slot0_cell=5, first_pt=6,
+          box_x0=7, box_y0=8, box_z0=9, box_x1=10, box_y1=11, box_z1=12, sphere_r2=13)
 QC = dict(n_cand=0, n_valid=1, n_pairs=2, R1=3, R2=4, overflow=5)
 
 # every symbol include/pnb200.h declares (tests check that the .so exports all of them)
